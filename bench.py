@@ -49,7 +49,14 @@ def parse_args():
     ap.add_argument("--no-verify", action="store_true", help="skip the post-run proof check (oracle verifier with the real pairing)")
     ap.add_argument("--save-proof", default=None, help="write the hashed proof, the verifier key and the public data to this JSON file "
                                                        "(checked afterwards on a CPU by tests/verify_saved_proof.py)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write the proof of the last step of each timed region as DIR/proof.npy (device-resident "
+                         "instance) and DIR/proof_e2e.npy (host buffers): one float32 per proof byte.  Inputs and zk stream are seeded, so "
+                         "two builds run with the same arguments can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def measured_peaks():
@@ -206,7 +213,7 @@ def main():
     clocks.begin()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        m.prove(pk, None, zk)
+        proof_dev = m.prove(pk, None, zk)
         dev_ms.append(pk.timings()["Marlin::Prover"])  # CUDA events on the library's stream
     barrier()
     wall = time.perf_counter() - t0
@@ -229,6 +236,11 @@ def main():
     barrier()
     wall_e2e = time.perf_counter() - t0
     clocks.close()
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, blob in (("proof", proof_dev), ("proof_e2e", proof)):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), np.frombuffer(blob, dtype=np.uint8).astype(np.float32))
     # outside every timed region: a proof from a fresh zk stream, hashed, so that runs with different window sizes,
     # GPU counts or library builds can be compared byte for byte
     import hashlib
