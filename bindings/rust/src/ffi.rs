@@ -19,6 +19,10 @@ pub struct b2m_ck {
     _p: [u8; 0],
 }
 #[repr(C)]
+pub struct b2m_verifier {
+    _p: [u8; 0],
+}
+#[repr(C)]
 pub struct b2m_matrix {
     pub row_ptr: *const u64,
     pub col: *const u64,
@@ -100,4 +104,11 @@ extern "C" {
     pub fn b2m_index_comms(idx: *const b2m_index, out_xy: *mut u64) -> c_int;
     pub fn b2m_prove(idx: *mut b2m_index, formatted_input: *const u64, n_input: usize, witness: *const u64, n_witness: usize,
                      zk_rng: *mut b2m_rng, proof: *mut u8, cap: usize, proof_len: *mut usize) -> c_int;
+    pub fn b2m_verifier_create(ctx: *mut b2m_ctx, curve: c_int, pc_variant: c_int, vk_tobytes: *const u8, vk_len: usize, g: *const u8,
+                               gamma_g: *const u8, h: *const u8, beta_h: *const u8, max_degree: usize, n_bounds: usize,
+                               bounds: *const u64, bound_points: *const u8, out: *mut *mut b2m_verifier) -> c_int;
+    pub fn b2m_verifier_destroy(ver: *mut b2m_verifier);
+    pub fn b2m_verify(ver: *mut b2m_verifier, n_proofs: usize, public_inputs: *const *const u64, n_inputs: *const usize,
+                      proofs: *const *const u8, proof_lens: *const usize, rng: *mut b2m_rng, verdicts: *mut c_int) -> c_int;
+    pub fn b2m_verify_timings(ver: *const b2m_verifier, json: *mut c_char, cap: usize) -> c_int;
 }

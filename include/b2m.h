@@ -267,6 +267,37 @@ int b2m_index_stage(b2m_index* idx, const uint64_t* formatted_input, size_t n_in
  * with the reference's own timer names (ark_std start_timer! labels, SURVEY.md section 5). */
 int b2m_prove_timings(const b2m_index* idx, char* json, size_t cap);
 
+/* ---- Level 3: verifier ABI -------------------------------------------------------------- */
+
+/* Per-proof outcome of b2m_verify. */
+enum { B2M_VERDICT_ACCEPT = 0, B2M_VERDICT_REJECT = 1, B2M_VERDICT_MALFORMED = 2 };
+
+typedef struct b2m_verifier b2m_verifier;
+
+/* The verifier key of `Marlin::verify` (reference src/lib.rs:315-433), device resident: the index_vk ToBytes image (what
+ * b2m_index_vk_bytes returns; absorbed verbatim by the transcript) plus the PC verifier key [U ark-poly-commit marlin_pc /
+ * sonic_pc VerifierKey]: g, gamma_g (G1) and h, beta_h (G2) as ark-serialize `serialize_uncompressed` bytes, the SRS's
+ * max_degree and the enforced degree bounds with, per bound, the MarlinKZG10 shift power powers_of_g[max_degree - bound] (G1,
+ * 2 * sizeof(Fq) bytes) or the SonicKZG10 beta^-(max_degree - bound) h (G2, 4 * sizeof(Fq) bytes), uncompressed, concatenated.
+ * h and beta_h are prepared once (Miller-loop line coefficients).  Errors: B2M_ERR_NON_SQUARE, B2M_ERR_DEGREE_TOO_LARGE
+ * (the index needs a larger supported degree), B2M_ERR_INVALID_ARG (a degree bound the index needs is not enforced --
+ * EquationHasDegreeBounds --, malformed bytes).  The verifier borrows the context. */
+int b2m_verifier_create(b2m_ctx* ctx, int curve, int pc_variant, const uint8_t* vk_tobytes, size_t vk_len, const uint8_t* g,
+                        const uint8_t* gamma_g, const uint8_t* h, const uint8_t* beta_h, size_t max_degree, size_t n_bounds,
+                        const uint64_t* bounds, const uint8_t* bound_points, b2m_verifier** out);
+void b2m_verifier_destroy(b2m_verifier* ver);
+
+/* `Marlin::verify` for n_proofs proofs of the verifier's index.  public_inputs[i]: n_inputs[i] Montgomery Fr (4 u64 each),
+ * without the leading one (as `R1CS.public_input()`); proofs[i]: `CanonicalSerialize` bytes of `Proof<F, PC>`.  rng supplies
+ * the 128-bit randomisers of the batched check [U ark-poly-commit check_combinations(.., rng)]: two per proof, then one per
+ * proof for the batch fold.  verdicts[i] = B2M_VERDICT_ACCEPT / REJECT / MALFORMED (unparsable bytes, a point off the curve or
+ * outside the prime-order subgroup, an evaluation >= r); a proof never affects another's verdict.  The return code is not
+ * B2M_OK only for misuse (null arguments, an unreduced public input) or CUDA errors. */
+int b2m_verify(b2m_verifier* ver, size_t n_proofs, const uint64_t* const* public_inputs, const size_t* n_inputs,
+               const uint8_t* const* proofs, const size_t* proof_lens, b2m_rng* rng, int* verdicts);
+/* Per-stage times of the last b2m_verify (milliseconds; device stages from CUDA events, "transcript" on the host). */
+int b2m_verify_timings(const b2m_verifier* ver, char* json, size_t cap);
+
 #ifdef __cplusplus
 }
 #endif

@@ -13,6 +13,7 @@ CURVE_BN254 = 1
 PC_MARLIN_KZG10 = 0
 PC_SONIC_KZG10 = 1
 RNG_CHACHA8, RNG_CHACHA12, RNG_CHACHA20 = 8, 12, 20
+VERDICT_ACCEPT, VERDICT_REJECT, VERDICT_MALFORMED = 0, 1, 2
 
 # (Fr u64 limbs, Fq u64 limbs) per curve id
 LIMBS = {CURVE_BLS12_381: (4, 6), CURVE_BN254: (4, 4)}
@@ -97,6 +98,11 @@ def lib():
             L.b2m_index_stage.argtypes = [vp, vp, sz, vp, sz]
             L.b2m_prove.argtypes = [vp, vp, sz, vp, sz, P(Rng), vp, sz, P(sz)]
             L.b2m_prove_timings.argtypes = [vp, ctypes.c_char_p, sz]
+        L.b2m_verifier_create.argtypes = [vp, ci, ci, vp, sz, vp, vp, vp, vp, sz, sz, vp, vp, P(vp)]
+        L.b2m_verifier_destroy.argtypes = [vp]
+        L.b2m_verifier_destroy.restype = None
+        L.b2m_verify.argtypes = [vp, sz, vp, vp, vp, vp, P(Rng), vp]
+        L.b2m_verify_timings.argtypes = [vp, ctypes.c_char_p, sz]
         _lib = L
     return _lib
 

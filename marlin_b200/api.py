@@ -3,12 +3,15 @@
 F in {BLS12-381 Fr, BN254 Fr}, PC in {MarlinKZG10, SonicKZG10}, FS = SimpleHashFiatShamirRng<Blake2s, ChaChaRng>.
 Every call lands in libb2m.so (include/b2m.h); nothing here computes on the CPU beyond marshalling.
 
-`verify` is not accelerated and not shipped by this package (SURVEY.md section 8f-2); proofs are
-`CanonicalSerialize` bytes that the reference's `Marlin::verify` consumes.
+`Marlin::verify` [reference src/lib.rs:315-433] is `Marlin.verify` / `Marlin.batch_verify` against a device-resident
+`VerifierKey` (b2m_verifier): compressed points are decoded and subgroup-checked on the GPU, the Fiat-Shamir transcripts are
+replayed on host threads, and a whole batch is folded into one pairing product checked on the GPU.  Proofs are
+`CanonicalSerialize` bytes, the same bytes the reference's `Marlin::verify` consumes.
 """
 import ctypes
 import json
 import os
+import struct
 
 import numpy as np
 
@@ -165,6 +168,38 @@ class IndexProverKey:
         if self.handle:
             _lib.lib().b2m_index_destroy(self.handle)
             self.handle = None
+
+
+class VerifierKey:
+    """`Marlin::verify`'s key on the device (b2m_verifier): the index_vk ToBytes image, the six index commitments, g, gamma g,
+    prepared h and beta h, and the enforced degree bounds with their shift powers (MarlinKZG10) or beta^-(D - d) h (SonicKZG10)."""
+
+    def __init__(self, ctx, curve_id, pc, handle, vk_bytes):
+        self.ctx, self.curve_id, self.pc, self.handle, self.vk_bytes = ctx, curve_id, pc, handle, vk_bytes
+
+    def timings(self):
+        """Per-stage times (ms) of the last verification with this key."""
+        buf = ctypes.create_string_buffer(4096)
+        _lib.check(_lib.lib().b2m_verify_timings(self.handle, buf, 4096))
+        return json.loads(buf.value.decode() or "{}")
+
+    def close(self):
+        if self.handle:
+            _lib.lib().b2m_verifier_destroy(self.handle)
+            self.handle = None
+
+
+def _pow2_at_least(n):
+    s = 1
+    while s < n:
+        s *= 2
+    return s
+
+
+def _index_bounds(vk_bytes):
+    """The degree bounds an index's proofs use: |H| - 2 (g_1) and |K| - 2 (g_2) [reference src/ahp/mod.rs get_degree_bounds]."""
+    _nv, nc, nnz = struct.unpack_from("<QQQ", vk_bytes, 0)
+    return sorted({_pow2_at_least(nc) - 2, _pow2_at_least(nnz) - 2})
 
 
 def max_degree(num_constraints, num_variables, num_non_zero):
@@ -377,3 +412,95 @@ class Marlin:
         inst = np.ascontiguousarray(r1cs.instance)
         wit = np.ascontiguousarray(r1cs.witness)
         _lib.check(_lib.lib().b2m_index_stage(index_pk.handle, _lib.ptr(inst), len(inst), _lib.ptr(wit), len(wit)))
+
+    # -- verify ----------------------------------------------------------------------------------------
+    def _verifier(self, vk_bytes, max_degree_, g, gamma_g, h, beta_h, bounds, bound_points):
+        L = _lib.lib()
+        out = ctypes.c_void_p()
+        b = np.asarray(bounds, dtype=np.uint64)
+        pts = np.frombuffer(b"".join(bound_points), dtype=np.uint8)
+        buf = lambda x: np.frombuffer(bytes(x), dtype=np.uint8)  # noqa: E731
+        vk, g_, gg, h_, bh = buf(vk_bytes), buf(g), buf(gamma_g), buf(h), buf(beta_h)
+        _lib.check(L.b2m_verifier_create(self.ctx.handle, self.curve_id, self.pc, _lib.ptr(vk), len(vk), _lib.ptr(g_), _lib.ptr(gg), _lib.ptr(h_),
+                                         _lib.ptr(bh), max_degree_, len(b), _lib.ptr(b) if len(b) else None, _lib.ptr(pts) if len(pts) else None,
+                                         ctypes.byref(out)))
+        return VerifierKey(self.ctx, self.curve_id, self.pc, out, bytes(vk_bytes))
+
+    def verifier_key(self, pk):
+        """The verifier key of an index made by `index` (reference `IndexVerifierKey` + the trimmed PC verifier key).  The G2 half
+        comes from the SRS's trapdoor (a test SRS) or from the file it was loaded from, as in `UniversalSRS.save`."""
+        from . import srsfile
+        srs = pk.srs
+        L = _lib.lib()
+        cid = self.curve_id
+        md = srs.max_degree
+        bounds = _index_bounds(pk.vk_bytes)
+        g1 = 2 * srsfile.fq_bytes(cid)
+
+        def g1_bytes(limbs):
+            limbs = np.ascontiguousarray(np.asarray(limbs, dtype=np.uint64).reshape(-1, 2 * _lib.LIMBS[cid][1]))
+            out = np.zeros(len(limbs) * g1, dtype=np.uint8)
+            _lib.check(L.b2m_g1_to_uncompressed(self.ctx.handle, cid, _lib.ptr(limbs), len(limbs), _lib.ptr(out)))
+            return out.tobytes()
+
+        if srs.trapdoor is not None:
+            h, beta_h, neg = srsfile.g2_setup(cid, fields.FR_MODULUS[cid], srs.trapdoor[0], md, bounds)
+        elif srs.g2 is not None:
+            h, beta_h, neg = srs.g2
+        else:
+            raise ValueError("this SRS has no G2 half (neither a trapdoor nor a source file)")
+        g = g1_bytes(srs.powers_limbs[0])
+        gamma_g = g1_bytes(srs.gamma_limbs[list(srs.gamma_indices).index(0)])
+        if self.pc == _lib.PC_MARLIN_KZG10:
+            points = [g1_bytes(srs.powers_limbs[md - d]) for d in bounds]
+        else:
+            points = [neg[md - d] for d in bounds]
+        return self._verifier(pk.vk_bytes, md, g, gamma_g, h, beta_h, bounds, points)
+
+    def verifier_key_from_files(self, srs_path, index_vk_tobytes):
+        """The verifier key from public data only: an SRS file (marlin_b200/srsfile.py layout) and the index_vk ToBytes image."""
+        from . import srsfile
+        d = srsfile.read_srs(srs_path)
+        if d["curve_id"] != self.curve_id:
+            raise ValueError(f"{srs_path} holds curve {d['curve_id']}, this Marlin instance is curve {self.curve_id}")
+        g1 = 2 * srsfile.fq_bytes(self.curve_id)
+        md = len(d["powers"]) // g1 - 1
+        bounds = _index_bounds(index_vk_tobytes)
+        if self.pc == _lib.PC_MARLIN_KZG10:
+            points = [d["powers"][(md - b) * g1:(md - b + 1) * g1] for b in bounds]
+        else:
+            missing = [b for b in bounds if md - b not in d["neg_powers"]]
+            if missing:
+                raise ValueError(f"{srs_path} holds no beta^-(D - d) h for the degree bounds {missing}")
+            points = [d["neg_powers"][md - b] for b in bounds]
+        return self._verifier(bytes(index_vk_tobytes), md, d["powers"][:g1], d["gamma"][0], d["h"], d["beta_h"], bounds, points)
+
+    def batch_verify(self, vk, items, rng=None):
+        """`Marlin::verify` [reference src/lib.rs:315-433] for [(public_input, proof_bytes), ...] of one index -> [bool].  The public
+        input is canonical ints without the leading one (`R1CS.public_input()`).  rng: the randomisers of the batched pairing check
+        (ZkRng / CallbackRng); None draws a fresh ChaCha stream seeded from os.urandom."""
+        L = _lib.lib()
+        n = len(items)
+        if n == 0:
+            return []
+        rng = rng or ZkRng()
+        r = fields.FR_MODULUS[self.curve_id]
+        ins, proofs = [], []
+        for pi, proof in items:
+            vals = [int(v) for v in pi]
+            if any(v < 0 or v >= r for v in vals):
+                raise ValueError("public input element out of range")
+            ins.append(_lib.ints_to_limbs([fields.fr_to_mont(self.curve_id, v) for v in vals], 4) if vals else np.zeros((0, 4), dtype=np.uint64))
+            proofs.append(np.frombuffer(bytes(proof), dtype=np.uint8) if len(proof) else np.zeros(1, dtype=np.uint8))
+        in_ptrs = (ctypes.c_void_p * n)(*[a.ctypes.data if len(a) else None for a in ins])
+        n_in = (ctypes.c_size_t * n)(*[len(a) for a in ins])
+        pr_ptrs = (ctypes.c_void_p * n)(*[a.ctypes.data for a in proofs])
+        pr_len = (ctypes.c_size_t * n)(*[len(p) for _, p in items])
+        verdicts = (ctypes.c_int * n)()
+        _lib.check(L.b2m_verify(vk.handle, n, in_ptrs, n_in, pr_ptrs, pr_len, ctypes.byref(rng.c), verdicts))
+        self.last_verdicts = [int(v) for v in verdicts]
+        return [v == _lib.VERDICT_ACCEPT for v in self.last_verdicts]
+
+    def verify(self, vk, public_input, proof, rng=None):
+        """`Marlin::verify` for one proof -> bool."""
+        return self.batch_verify(vk, [(public_input, proof)], rng)[0]

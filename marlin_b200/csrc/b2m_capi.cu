@@ -2,6 +2,7 @@
 // The prover-level entry points live in prover.cu.
 #include "capi_types.cuh"
 #include "prover.cuh"
+#include "verify.cuh"
 #include "comm.cuh"
 #include <algorithm>
 #include "g2_host.hpp"
@@ -474,6 +475,58 @@ int b2m_prove_timings(const b2m_index* idx, char* json, size_t cap) {
   return guard([&] {
     B2M_REQUIRE(idx && json && cap > 0, B2M_ERR_INVALID_ARG, "null argument");
     snprintf(json, cap, "%s", idx->impl->timings_json.c_str());
+  });
+}
+
+// ---- Level 3 ----------------------------------------------------------------------------------
+struct b2m_verifier {
+  b2m_ctx* ctx;
+  std::unique_ptr<VerifierBase> impl;
+};
+
+int b2m_verifier_create(b2m_ctx* ctx, int curve, int pc_variant, const uint8_t* vk_tobytes, size_t vk_len, const uint8_t* g,
+                        const uint8_t* gamma_g, const uint8_t* h, const uint8_t* beta_h, size_t max_degree, size_t n_bounds,
+                        const uint64_t* bounds, const uint8_t* bound_points, b2m_verifier** out) {
+  return guard([&] {
+    B2M_REQUIRE(ctx && vk_tobytes && g && gamma_g && h && beta_h && out && (n_bounds == 0 || (bounds && bound_points)), B2M_ERR_INVALID_ARG,
+                "null argument");
+    B2M_REQUIRE(pc_variant == B2M_PC_MARLIN_KZG10 || pc_variant == B2M_PC_SONIC_KZG10, B2M_ERR_INVALID_ARG, "unknown PC variant");
+    ctx->cx.use();
+    std::unique_ptr<b2m_verifier> v(new b2m_verifier);
+    v->ctx = ctx;
+    if (curve == B2M_CURVE_BLS12_381)
+      v->impl.reset(make_verifier_bls(ctx->cx, pc_variant, vk_tobytes, vk_len, g, gamma_g, h, beta_h, max_degree, n_bounds, bounds, bound_points));
+    else if (curve == B2M_CURVE_BN254)
+      v->impl.reset(make_verifier_bn(ctx->cx, pc_variant, vk_tobytes, vk_len, g, gamma_g, h, beta_h, max_degree, n_bounds, bounds, bound_points));
+    else
+      throw Error(B2M_ERR_INVALID_ARG, "unknown curve id");
+    *out = v.release();
+    ctx->children++;
+  });
+}
+
+void b2m_verifier_destroy(b2m_verifier* ver) {
+  if (!ver) return;
+  b2m_ctx* ctx = ver->ctx;
+  ctx->cx.use();
+  cudaStreamSynchronize(ctx->cx.stream);
+  delete ver;
+  if (--ctx->children == 0 && ctx->dead) b2m_release_ctx(ctx);
+}
+
+int b2m_verify(b2m_verifier* ver, size_t n_proofs, const uint64_t* const* public_inputs, const size_t* n_inputs, const uint8_t* const* proofs,
+               const size_t* proof_lens, b2m_rng* rng, int* verdicts) {
+  return guard([&] {
+    B2M_REQUIRE(ver, B2M_ERR_INVALID_ARG, "null verifier");
+    ver->ctx->cx.use();
+    ver->impl->verify(n_proofs, public_inputs, n_inputs, proofs, proof_lens, rng, verdicts);
+  });
+}
+
+int b2m_verify_timings(const b2m_verifier* ver, char* json, size_t cap) {
+  return guard([&] {
+    B2M_REQUIRE(ver && json && cap > 0, B2M_ERR_INVALID_ARG, "null argument");
+    snprintf(json, cap, "%s", ver->impl->timings_json.c_str());
   });
 }
 

@@ -4,37 +4,15 @@
 // the same limb code as the device (field.cuh compiled for the host), written out in ark-serialize's uncompressed form so that
 // an SRS file made here can be loaded by arkworks (tools/replay_rs).
 //
-// Fq2 = Fq[u] / (u^2 + 1) for both supported curves; E'(Fq2): y^2 = x^3 + b' (the formulas below never need b').
+// Fq2 (pairing.cuh) = Fq[u] / (u^2 + 1) for both supported curves; E'(Fq2): y^2 = x^3 + b' (the formulas below never need b').
 #pragma once
 #include <cstdint>
 #include <cstring>
 #include <vector>
 
-#include "field.cuh"
+#include "pairing.cuh"  // Fq2
 
 namespace b2m {
-
-template <class Fq>
-struct Fq2 {
-  Fq c0, c1;
-  static Fq2 zero() { return Fq2{Fq::zero(), Fq::zero()}; }
-  static Fq2 one() { return Fq2{Fq::one(), Fq::zero()}; }
-  bool is_zero() const { return c0.is_zero() && c1.is_zero(); }
-  bool operator==(const Fq2& o) const { return c0 == o.c0 && c1 == o.c1; }
-  friend Fq2 operator+(const Fq2& a, const Fq2& b) { return Fq2{a.c0 + b.c0, a.c1 + b.c1}; }
-  friend Fq2 operator-(const Fq2& a, const Fq2& b) { return Fq2{a.c0 - b.c0, a.c1 - b.c1}; }
-  friend Fq2 operator*(const Fq2& a, const Fq2& b) {  // Karatsuba, u^2 = -1
-    const Fq v0 = a.c0 * b.c0, v1 = a.c1 * b.c1;
-    return Fq2{v0 - v1, (a.c0 + a.c1) * (b.c0 + b.c1) - v0 - v1};
-  }
-  Fq2 sqr() const { return (*this) * (*this); }
-  Fq2 dbl() const { return Fq2{c0.dbl(), c1.dbl()}; }
-  Fq2 neg() const { return Fq2{c0.neg(), c1.neg()}; }
-  Fq2 inverse() const {  // (c0 - c1 u) / (c0^2 + c1^2)
-    const Fq n = (c0.sqr() + c1.sqr()).inverse();
-    return Fq2{c0 * n, (c1 * n).neg()};
-  }
-};
 
 template <class Fq>
 struct G2Jac {  // Jacobian: (X / Z^2, Y / Z^3); infinity: Z = 0

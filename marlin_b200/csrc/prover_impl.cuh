@@ -22,6 +22,7 @@
 #include "prover.cuh"
 #include "comm.cuh"
 #include "scan.cuh"
+#include "verify_core.cuh"
 
 namespace b2m {
 
@@ -742,19 +743,11 @@ struct MarlinIndex : IndexBase {
       c.l[0] = (uint32_t)lo; c.l[1] = (uint32_t)(lo >> 32); c.l[2] = (uint32_t)hi; c.l[3] = (uint32_t)(hi >> 32);
       xi = Fr::from_canonical(c);
     }
-    // linear-combination coefficients [reference mod.rs:145-213]
-    Fr r_alpha_at_beta = (v_h_alpha - v_h_beta) * (alpha - beta).inverse();
-    if (alpha == beta) r_alpha_at_beta = Fr::from_u64(H) * alpha.pow_u64(H - 1);
-    Fr v_x_beta = beta.pow_u64(X) - one;
-    Fr c_za = r_alpha_at_beta * (eta_a + eta_c * zb_at_beta);
-    Fr c_w = (t_at_beta * v_x_beta).neg();
-    Fr c_h1 = v_h_beta.neg();
-    Fr v_k_gamma = gamma.pow_u64(K) - one;
-    Fr k_inv = Fr::from_u64(K).inverse();
-    Fr bscale = gamma * g2_at_gamma + t_at_beta * k_inv;
-    // inner_sumcheck = v (eta_a a_val + eta_b b_val + eta_c c_val) - bscale (-alpha row - beta col + row_col) - v_K(gamma) h_2
-    Fr ci_a = ea_v, ci_b = eb_v, ci_c = ec_v;
-    Fr ci_row = bscale * alpha, ci_col = bscale * beta, ci_rc = bscale.neg(), ci_h2 = v_k_gamma.neg();
+    // linear-combination coefficients [reference mod.rs:145-213], shared with the verifier (verify_core.cuh); the prover skips the
+    // constant terms, so x_hat(beta) is not needed here
+    const LcCoeffs<Fr> lc = lc_coefficients(Challenges<Fr>{alpha, eta_a, eta_b, eta_c, beta, gamma}, evals, H, K, X, Fr::zero());
+    const Fr c_za = lc.za, c_w = lc.w, c_h1 = lc.h1;
+    const Fr ci_a = lc.a, ci_b = lc.b, ci_c = lc.c, ci_row = lc.row, ci_col = lc.col, ci_rc = lc.rc, ci_h2 = lc.h2;
     tm.end(t_ev);
 
     // ---- open_combinations [U ark-poly-commit marlin_pc / sonic_pc; SURVEY.md App. B] ---------------------
