@@ -47,6 +47,7 @@ struct Ctx {
   int sm_count = 148;
   cudaStream_t stream = nullptr;  // the stream every helper launches on (see StreamSwap)
   cudaStream_t side = nullptr;    // second stream: sort of the next MSM while the current one accumulates
+  cudaStream_t lane1 = nullptr;   // third stream: Msm::run_batch's second bucket-pass lane (`stream` is the first)
   cudaMemPool_t pool = nullptr;
   // multi-GPU MSM sharding (comm.cuh): rank / world of this process and its ncclComm_t
   int rank = 0, world = 1;
@@ -106,11 +107,13 @@ struct Ctx {
     sm_count = prop.multiProcessorCount;
     B2M_CUDA(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
     B2M_CUDA(cudaStreamCreateWithFlags(&side, cudaStreamNonBlocking));
+    B2M_CUDA(cudaStreamCreateWithFlags(&lane1, cudaStreamNonBlocking));
     B2M_CUDA(cudaDeviceGetDefaultMemPool(&pool, dev));
     unsigned long long thr = ~0ull;  // keep freed blocks cached in the pool
     B2M_CUDA(cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thr));
   }
   ~Ctx() {
+    if (lane1) cudaStreamDestroy(lane1);
     if (side) cudaStreamDestroy(side);
     if (stream) cudaStreamDestroy(stream);
   }

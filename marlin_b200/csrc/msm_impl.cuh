@@ -6,6 +6,8 @@
 #include "msm_affine.cuh"
 #include "comm.cuh"
 
+#include <algorithm>
+
 namespace b2m {
 
 template <class Fq>
@@ -772,24 +774,30 @@ void Msm<Fr, Fq>::run_batch(const MsmJob<Fr, Fq>* jobs_in, int nj) {
   const size_t L = (size_t)1 << cbits, R = (size_t)1 << rbits;
   DBuf<XYZZ<Fq>> buckets(cx, (size_t)nj * B);
   {
-    // Software pipeline over the jobs: the counting sort of job j + 1 (memory / atomic bound, ~40 registers per
-    // thread) runs on the side stream while job j's bucket pass (integer-ALU bound, 2 CTAs/SM) runs on the main
-    // stream; sort buffers are double-buffered and the two streams are chained with events.
+    // Software pipeline over the jobs on three streams.  The counting sorts (memory / atomic bound, ~40 registers per thread)
+    // run ahead on the side stream.  The bucket passes (levels, accumulate, stitch: integer-ALU bound) alternate between two
+    // lanes, cx.stream and cx.lane1, so that the stages of one pass that leave most SMs idle -- the batch inversions, the
+    // short plan / count / scan launches, the stitch, the partial last wave of every kernel -- run under the other pass's
+    // throughput kernels.  Jobs are issued largest first: the k-th issued job, order[k], sorts into slot k % slots and runs
+    // its bucket pass on lane k % 2.  Every job writes its own bucket array, so neither order nor lane changes a result.
+    // Sort slots: a slot is read by its job's bucket pass (level 0, or accumulate and stitch) until the pass ends (ev_acc).
+    // With two passes in flight, three slots let the sort of job k + 2 run while k and k + 1 are still on the lanes; the
+    // sort of k + 3 waits for the end of k.  Everything else a bucket pass writes exists once per lane (LaneScratch).
     const size_t max_refs = (size_t)W * max_n;
     const size_t max_threads = (max_refs + MSM_Q_MIN - 1) / MSM_Q_MIN + 256;  // launches round up to whole blocks
-    DBuf<uint32_t> digits[2], hist[2], offsets[2], cursor[2];
-    DBuf<uint2> sorted[2];
-    const int slots = nj > 1 ? 2 : 1;
+    const int slots = std::min(nj, 3), lanes = std::min(nj, 2);
+    const cudaStream_t lane_stream[2] = {cx.stream, cx.lane1};
+    int order[MSM_MAX_BATCH];
+    for (int j = 0; j < nj; j++) order[j] = j;
+    std::stable_sort(order, order + nj, [&](int a, int b) { return jobs[a].n + jobs[a].n2 > jobs[b].n + jobs[b].n2; });
+    DBuf<uint32_t> digits[3], hist[3], offsets[3], cursor[3];
+    DBuf<uint2> sorted[3];
     for (int s = 0; s < slots; s++) {
       digits[s] = DBuf<uint32_t>(cx, max_refs); hist[s] = DBuf<uint32_t>(cx, B + 1); offsets[s] = DBuf<uint32_t>(cx, B + 1);
       cursor[s] = DBuf<uint32_t>(cx, B); sorted[s] = DBuf<uint2>(cx, max_refs);
     }
-    DBuf<uint32_t> part_bkt(cx, 2 * max_threads), n_long(cx, 4);  // queued long-run entries, second-stage entries, chunk slots, short runs
     const uint32_t long_cap = 1u << 18;
     const uint32_t chunk_cap = (uint32_t)(4 * max_threads / MSM_RUN_CHUNK + 4);  // every chunk but a run's last covers MSM_RUN_CHUNK slots
-    DBuf<MsmLongRun> long_runs(cx, long_cap), short_runs(cx, long_cap), final_runs(cx, chunk_cap);
-    DBuf<XYZZ<Fq>> chunk_pt(cx, chunk_cap);
-    DBuf<XYZZ<Fq>> part_pt(cx, 2 * max_threads);
     // batched-affine levels (msm_affine.cuh): level l has at most bound[l] points
     const int LV = max_refs >= affine_min_refs ? affine_levels : 0;  // (the largest job of the batch decides the buffers)
     // the level-0 plan packs (window * stride + index) | sign << 31 into 32 bits (msm_affine.cuh aff_plan_thread)
@@ -798,41 +806,62 @@ void Msm<Fr, Fq>::run_batch(const MsmJob<Fr, Fq>* jobs_in, int nj) {
     size_t bound[MSM_MAX_AFFINE_LEVELS + 1];
     bound[0] = max_refs;
     for (int l = 1; l <= LV; l++) bound[l] = (bound[l - 1] + B) / 2 + 1;
-    DBuf<Affine<Fq>> lvl_pts[2];
-    DBuf<uint32_t> lvl_off[2], lvl_cnt;
-    DBuf<uint2> lvl_refs;
-    DBuf<uint4> lvl_meta;
-    DBuf<Fq> lvl_pref, lvl_inv;
-    if (LV > 0) {
-      lvl_pts[0] = DBuf<Affine<Fq>>(cx, bound[1]);
-      if (LV > 1) lvl_pts[1] = DBuf<Affine<Fq>>(cx, bound[2]);
-      lvl_off[0] = DBuf<uint32_t>(cx, B + 1); lvl_off[1] = DBuf<uint32_t>(cx, B + 1); lvl_cnt = DBuf<uint32_t>(cx, B + 1);
-      lvl_refs = DBuf<uint2>(cx, bound[LV]);
-      const size_t T_max = (size_t)std::max(affine_T, affine_T_upper), T_min = (size_t)std::min(affine_T, affine_T_upper);
-      const size_t slots_l0 = T_max * ((bound[1] + T_max - 1) / T_max + 128);  // >= T * nthreads at every level, for either mapping
-      lvl_meta = DBuf<uint4>(cx, slots_l0);
-      lvl_pref = DBuf<Fq>(cx, slots_l0);
-      lvl_inv = DBuf<Fq>(cx, slots_l0 / T_min + 256);
+    const size_t T_max = (size_t)std::max(affine_T, affine_T_upper), T_min = (size_t)std::min(affine_T, affine_T_upper);
+    const size_t slots_l0 = LV > 0 ? T_max * ((bound[1] + T_max - 1) / T_max + 128) : 0;  // >= T * nthreads at every level, for either mapping
+    struct LaneScratch {
+      DBuf<uint32_t> part_bkt, n_long;  // n_long: queued long-run entries, second-stage entries, chunk slots, short runs
+      DBuf<MsmLongRun> long_runs, short_runs, final_runs;
+      DBuf<XYZZ<Fq>> chunk_pt, part_pt;
+      DBuf<Affine<Fq>> lvl_pts[2];
+      DBuf<uint32_t> lvl_off[2], lvl_cnt;
+      DBuf<uint2> lvl_refs;
+      DBuf<uint4> lvl_meta;
+      DBuf<Fq> lvl_pref, lvl_inv;
+    } lane[2];
+    for (int i = 0; i < lanes; i++) {
+      LaneScratch& ls = lane[i];
+      ls.part_bkt = DBuf<uint32_t>(cx, 2 * max_threads); ls.n_long = DBuf<uint32_t>(cx, 4);
+      ls.long_runs = DBuf<MsmLongRun>(cx, long_cap); ls.short_runs = DBuf<MsmLongRun>(cx, long_cap);
+      ls.final_runs = DBuf<MsmLongRun>(cx, chunk_cap);
+      ls.chunk_pt = DBuf<XYZZ<Fq>>(cx, chunk_cap);
+      ls.part_pt = DBuf<XYZZ<Fq>>(cx, 2 * max_threads);
+      if (LV > 0) {
+        ls.lvl_pts[0] = DBuf<Affine<Fq>>(cx, bound[1]);
+        if (LV > 1) ls.lvl_pts[1] = DBuf<Affine<Fq>>(cx, bound[2]);
+        ls.lvl_off[0] = DBuf<uint32_t>(cx, B + 1); ls.lvl_off[1] = DBuf<uint32_t>(cx, B + 1); ls.lvl_cnt = DBuf<uint32_t>(cx, B + 1);
+        ls.lvl_refs = DBuf<uint2>(cx, bound[LV]);
+        ls.lvl_meta = DBuf<uint4>(cx, slots_l0);
+        ls.lvl_pref = DBuf<Fq>(cx, slots_l0);
+        ls.lvl_inv = DBuf<Fq>(cx, slots_l0 / T_min + 256);
+      }
     }
     buckets.zero();  // empty buckets are never written: all-zero XYZZ is the point at infinity
-    cudaEvent_t ev_ready, ev_sorted[MSM_MAX_BATCH], ev_acc[MSM_MAX_BATCH];
+    // events are indexed by issue position k
+    cudaEvent_t ev_ready, ev_join, ev_sorted[MSM_MAX_BATCH], ev_acc[MSM_MAX_BATCH];
     B2M_CUDA(cudaEventCreateWithFlags(&ev_ready, cudaEventDisableTiming));
-    for (int j = 0; j < nj; j++) {
-      B2M_CUDA(cudaEventCreateWithFlags(&ev_sorted[j], cudaEventDisableTiming));
-      B2M_CUDA(cudaEventCreateWithFlags(&ev_acc[j], cudaEventDisableTiming));
+    B2M_CUDA(cudaEventCreateWithFlags(&ev_join, cudaEventDisableTiming));
+    for (int k = 0; k < nj; k++) {
+      B2M_CUDA(cudaEventCreateWithFlags(&ev_sorted[k], cudaEventDisableTiming));
+      B2M_CUDA(cudaEventCreateWithFlags(&ev_acc[k], cudaEventDisableTiming));
     }
     B2M_CUDA(cudaEventRecord(ev_ready, cx.stream));  // buffers exist (stream-ordered allocation) and inputs are final
     B2M_CUDA(cudaStreamWaitEvent(cx.side, ev_ready, 0));
-    for (int j = 0; j < nj; j++) {
+    if (lanes > 1) B2M_CUDA(cudaStreamWaitEvent(cx.lane1, ev_ready, 0));
+    for (int k = 0; k < nj; k++) {
+      const int j = order[k];
       const size_t n = jobs[j].n, nt = jobs[j].n + jobs[j].n2;
-      const int s = j % slots;
+      const int s = k % slots;
+      LaneScratch& ls = lane[k % 2];
+      StreamSwap on_lane(cx, lane_stream[k % 2]);  // this job's DBufs, scans and spans follow its lane
       if (nt == 0) {
-        B2M_CUDA(cudaEventRecord(ev_acc[j], cx.stream));
+        // no sort and no pass; ev_acc[k] still has to mean "slot s is free": the slot's last user may be on the other lane
+        if (k >= slots) B2M_CUDA(cudaStreamWaitEvent(cx.stream, ev_acc[k - slots], 0));
+        B2M_CUDA(cudaEventRecord(ev_acc[k], cx.stream));
         continue;
       }
       {
         StreamSwap on_side(cx, cx.side);
-        if (j >= slots) B2M_CUDA(cudaStreamWaitEvent(cx.side, ev_acc[j - slots], 0));  // the slot's previous user is done
+        if (k >= slots) B2M_CUDA(cudaStreamWaitEvent(cx.side, ev_acc[k - slots], 0));  // the slot's previous user is done
         hist[s].zero();
         size_t sp0 = cx.span_begin("msm_sort", (double)n);
         msm_digits_kernel<Fr><<<div_up(nt, 256), 256, 0, cx.stream>>>(jobs[j].scalars, jobs[j].scalar_stride, jobs[j].scalars2, jobs[j].mont, n, nt, c, W,
@@ -845,9 +874,9 @@ void Msm<Fr, Fq>::run_batch(const MsmJob<Fr, Fq>* jobs_in, int nj) {
         B2M_CHECK_LAUNCH();
         cx.launches += 2;
         cx.span_end(sp0);
-        B2M_CUDA(cudaEventRecord(ev_sorted[j], cx.side));
+        B2M_CUDA(cudaEventRecord(ev_sorted[k], cx.side));
       }
-      B2M_CUDA(cudaStreamWaitEvent(cx.stream, ev_sorted[j], 0));
+      B2M_CUDA(cudaStreamWaitEvent(cx.stream, ev_sorted[k], 0));
       // source of the XYZZ bucket pass: the sorted references into the window tables, or -- after LV batched-affine
       // levels -- the last level's points with one reference each
       const Affine<Fq>* src_tables = tables.p;
@@ -861,21 +890,21 @@ void Msm<Fr, Fq>::run_batch(const MsmJob<Fr, Fq>* jobs_in, int nj) {
         for (int l = 1; l <= LV; l++) bound[l] = (bound[l - 1] + B) / 2 + 1;
         const uint32_t* off_in = offsets[s].p;
         for (int l = 0; l < LV; l++) {
-          uint32_t* off_out = lvl_off[l & 1].p;
-          msm_level_counts_kernel<<<div_up((size_t)B + 1, 256), 256, 0, cx.stream>>>(off_in, B, lvl_cnt.p);
+          uint32_t* off_out = ls.lvl_off[l & 1].p;
+          msm_level_counts_kernel<<<div_up((size_t)B + 1, 256), 256, 0, cx.stream>>>(off_in, B, ls.lvl_cnt.p);
           B2M_CHECK_LAUNCH();
           cx.launches++;
-          exclusive_scan_u32(cx, lvl_cnt.p, off_out, (size_t)B + 1);
+          exclusive_scan_u32(cx, ls.lvl_cnt.p, off_out, (size_t)B + 1);
           const uint32_t lane_step = affine_map ? 32u : 1u;
           const size_t T_l = (size_t)(l == 0 ? affine_T : affine_T_upper);  // additions per thread (and per chain) at this level
           const uint32_t nthreads = (uint32_t)(lane_step * ((bound[l + 1] + (size_t)lane_step * T_l - 1) / ((size_t)lane_step * T_l)));
-          AffLevel<Fq> A{tables.p, stride, sorted[s].p, l > 0 ? lvl_pts[(l - 1) & 1].p : nullptr, off_in, off_out, B, lvl_pts[l & 1].p,
-                         l == LV - 1 ? lvl_refs.p : nullptr, lvl_pref.p, lvl_meta.p, (uint32_t)T_l, nthreads, lane_step, lvl_inv.p};
+          AffLevel<Fq> A{tables.p, stride, sorted[s].p, l > 0 ? ls.lvl_pts[(l - 1) & 1].p : nullptr, off_in, off_out, B, ls.lvl_pts[l & 1].p,
+                         l == LV - 1 ? ls.lvl_refs.p : nullptr, ls.lvl_pref.p, ls.lvl_meta.p, (uint32_t)T_l, nthreads, lane_step, ls.lvl_inv.p};
           if (l == 0)
             msm_affine_plan_kernel<Fq, true><<<div_up(nthreads, 256), 256, 0, cx.stream>>>(A);
           else
             msm_affine_plan_kernel<Fq, false><<<div_up(nthreads, 256), 256, 0, cx.stream>>>(A);
-          const Affine<Fq>* base = l == 0 ? tables.p : lvl_pts[(l - 1) & 1].p;
+          const Affine<Fq>* base = l == 0 ? tables.p : ls.lvl_pts[(l - 1) & 1].p;
           const unsigned grid = div_up(nthreads, 128);
           // Kernel variant (B2M_MSM_AFFINE_CTAS / _UPPER; every variant gives the same bytes, profiles/r02_level_kernel_notes.md):
           //   4 (default), 5: fused kernel, loads at use, compiled for that many resident CTAs per SM; 3: operands prefetched (3 CTAs/SM)
@@ -901,7 +930,7 @@ void Msm<Fr, Fq>::run_batch(const MsmJob<Fr, Fq>* jobs_in, int nj) {
             // split with the level-wide batch inversion between the two passes (21: plain addition pass at 4 CTAs/SM, 22: pipelined at 3)
             case 21: case 22:
               msm_affine_level_sp_kernel<Fq, 6, 3><<<grid, 128, 0, cx.stream>>>(A, base);
-              fq_batch_inverse_kernel<Fq><<<div_up(div_up(nthreads, 4), 128), 128, 0, cx.stream>>>(lvl_inv.p, nthreads);
+              fq_batch_inverse_kernel<Fq><<<div_up(div_up(nthreads, 4), 128), 128, 0, cx.stream>>>(ls.lvl_inv.p, nthreads);
               if (variant == 21) msm_affine_level_sp_kernel<Fq, 4, 2, false><<<grid, 128, 0, cx.stream>>>(A, base);
               else msm_affine_level_sp_kernel<Fq, 3, 2><<<grid, 128, 0, cx.stream>>>(A, base);
               cx.launches += 2;
@@ -914,10 +943,10 @@ void Msm<Fr, Fq>::run_batch(const MsmJob<Fr, Fq>* jobs_in, int nj) {
           off_in = off_out;
         }
         cx.span_end(spl);
-        src_tables = lvl_pts[(LV - 1) & 1].p;
+        src_tables = ls.lvl_pts[(LV - 1) & 1].p;
         src_stride = 0;
         src_off = off_in;
-        src_sorted = lvl_refs.p;
+        src_sorted = ls.lvl_refs.p;
         refs = bound[LV];
       }
       const uint32_t* src_ends = src_off + 1;   // buckets are contiguous: bucket b ends where b + 1 starts
@@ -932,31 +961,41 @@ void Msm<Fr, Fq>::run_batch(const MsmJob<Fr, Fq>* jobs_in, int nj) {
       if (q < (uint32_t)MSM_Q_MIN) q = MSM_Q_MIN;
       const size_t nthreads = (refs + q - 1) / q;
       msm_accumulate_kernel<Fq><<<div_up(nthreads, 128), 128, 0, cx.stream>>>(src_tables, src_stride, src_off, src_ends, src_sorted,
-                                                                               src_total, q, buckets.p + (size_t)j * B, part_pt.p,
-                                                                               part_bkt.p);
+                                                                               src_total, q, buckets.p + (size_t)j * B, ls.part_pt.p,
+                                                                               ls.part_bkt.p);
       B2M_CHECK_LAUNCH();
       cx.launches++;
       cx.span_end(sp);
       size_t sp1 = cx.span_begin("msm_stitch", (double)n);
-      n_long.zero();
-      msm_stitch_kernel<Fq><<<div_up(nthreads, 128), 128, 0, cx.stream>>>(part_pt.p, part_bkt.p, nthreads, q, src_off, src_ends,
-                                                                           buckets.p + (size_t)j * B, long_runs.p, final_runs.p, short_runs.p, n_long.p,
+      ls.n_long.zero();
+      msm_stitch_kernel<Fq><<<div_up(nthreads, 128), 128, 0, cx.stream>>>(ls.part_pt.p, ls.part_bkt.p, nthreads, q, src_off, src_ends,
+                                                                           buckets.p + (size_t)j * B, ls.long_runs.p, ls.final_runs.p, ls.short_runs.p, ls.n_long.p,
                                                                            long_cap, chunk_cap);
-      msm_stitch_short_kernel<Fq><<<2 * cx.sm_count, 128, 0, cx.stream>>>(part_pt.p, part_bkt.p, short_runs.p, n_long.p + 3, long_cap,
+      msm_stitch_short_kernel<Fq><<<2 * cx.sm_count, 128, 0, cx.stream>>>(ls.part_pt.p, ls.part_bkt.p, ls.short_runs.p, ls.n_long.p + 3, long_cap,
                                                                           buckets.p + (size_t)j * B);
-      msm_stitch_runs_kernel<Fq, false><<<4 * cx.sm_count, 128, 0, cx.stream>>>(part_pt.p, part_bkt.p, long_runs.p, n_long.p, long_cap,
-                                                                                buckets.p + (size_t)j * B, chunk_pt.p);
-      msm_stitch_runs_kernel<Fq, true><<<cx.sm_count, 128, 0, cx.stream>>>(part_pt.p, part_bkt.p, final_runs.p, n_long.p + 1, chunk_cap,
-                                                                           buckets.p + (size_t)j * B, chunk_pt.p);
+      msm_stitch_runs_kernel<Fq, false><<<4 * cx.sm_count, 128, 0, cx.stream>>>(ls.part_pt.p, ls.part_bkt.p, ls.long_runs.p, ls.n_long.p, long_cap,
+                                                                                buckets.p + (size_t)j * B, ls.chunk_pt.p);
+      msm_stitch_runs_kernel<Fq, true><<<cx.sm_count, 128, 0, cx.stream>>>(ls.part_pt.p, ls.part_bkt.p, ls.final_runs.p, ls.n_long.p + 1, chunk_cap,
+                                                                           buckets.p + (size_t)j * B, ls.chunk_pt.p);
       B2M_CHECK_LAUNCH();
       cx.launches += 4;
       cx.span_end(sp1);
-      B2M_CUDA(cudaEventRecord(ev_acc[j], cx.stream));
+      B2M_CUDA(cudaEventRecord(ev_acc[k], cx.stream));
+    }
+    if (lanes > 1) {
+      // Join lane 1 into cx.stream.  Every buffer of this block is freed at its closing brace below, on cx.stream (a DBuf is
+      // freed on the stream that is current when it is destroyed), and lane 1's scratch, the sort slots and `buckets` are
+      // read or written on lane 1: those frees, and the reduction after this block, are ordered behind lane 1's work only
+      // through this wait.  No buffer that lane 1 uses may be destroyed before this point.  (The side stream needs no join
+      // of its own: each of its sorts ends in an ev_sorted that a lane waits for.)
+      B2M_CUDA(cudaEventRecord(ev_join, cx.lane1));
+      B2M_CUDA(cudaStreamWaitEvent(cx.stream, ev_join, 0));
     }
     cudaEventDestroy(ev_ready);
-    for (int j = 0; j < nj; j++) {
-      cudaEventDestroy(ev_sorted[j]);
-      cudaEventDestroy(ev_acc[j]);
+    cudaEventDestroy(ev_join);
+    for (int k = 0; k < nj; k++) {
+      cudaEventDestroy(ev_sorted[k]);
+      cudaEventDestroy(ev_acc[k]);
     }
   }
   double units = 0;
